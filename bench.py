@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark: walker-steps/s of the red-blue walker update.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one full ensemble step (every walker proposed once = the P
@@ -18,8 +18,9 @@ before every step; ``e2e`` is the same metric through the public API
 ``EnsembleSampler.run_mcmc`` with pinned HOST buffers, copies inside the timed
 region (sharded: every rank moves only the rows it owns).  ``configs`` holds
 short runs of BASELINE.json's other configurations.  ``--impl reference`` times
-the UNMODIFIED reference package (``baseline/_ref``: ``vectorize=True`` and
-``multiprocessing.Pool``) on the host cores, with the numpy oracle port beside it.
+the UNMODIFIED reference package (``oracle/_ref``: ``vectorize=True`` and
+``multiprocessing.Pool``) on the host cores, with the numpy oracle port beside it,
+each over exactly ``--steps`` steps after ``--warmup``.
 """
 
 import argparse
@@ -39,8 +40,9 @@ if ROOT not in sys.path:
 
 METRIC = "walker-steps/sec (nwalkers x iters / s)"
 MODEL_SEED, INIT_SEED, SAMPLER_SEED = 20240, 20241, 0x656D636565B200
-REF_ZIP = os.path.join(ROOT, "baseline", "_ref", "emcee_reference.zip")
+REF_ZIP = os.path.join(ROOT, "oracle", "_ref", "emcee_reference.zip")
 FP64_PEAK_RECORDED = 37.0  # TFLOP/s, eb_microbench DMMA m8n8k4 (profiles/r01_fp64_microbench.txt)
+DUMP_BYTES, DUMP_SEED = 64 * 10**6, 0xD0  # --dump-outputs: size cap of all files together, walker-sample seed
 
 
 # --------------------------------------------------------------------------
@@ -145,6 +147,24 @@ class ClockSampler(object):
         return out
 
 
+def dump_outputs(dirname, coords, log_prob, naccepted):
+    """``--dump-outputs``: the ensemble state the timed steps left -- what ``run_mcmc`` hands its caller --
+    and the per-walker acceptance counts, as ``<dirname>/{coords,log_prob,naccepted}.npy`` (float64).  When
+    they would exceed DUMP_BYTES together, the same fixed seeded sample of walkers is taken from each and
+    its row numbers are written as ``walkers.npy``."""
+    out = {"coords": coords, "log_prob": log_prob, "naccepted": naccepted.astype(np.float64)}
+    n, d = coords.shape
+    per_walker = 8 * (d + 2)
+    if n * per_walker > DUMP_BYTES:
+        k = (DUMP_BYTES - 4096) // (per_walker + 8)  # 4096: room for the .npy headers
+        rows = np.sort(np.random.default_rng(DUMP_SEED).choice(n, k, replace=False))
+        out = {name: a[rows] for name, a in out.items()}
+        out["walkers"] = rows.astype(np.float64)
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(dirname, name + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
+
+
 def kernel_traffic(kernel):
     """DRAM bytes per launch of the dominant kernel from the committed `ncu --set full` capture
     (profiles/traffic.json, written by scripts/summarize_ncu.py), or None."""
@@ -180,7 +200,7 @@ def host_cores():
 
 
 # --------------------------------------------------------------------------
-# CPU arms (bench.py may execute oracle/ and baseline/_ref only here)
+# CPU arms (bench.py may execute oracle/ and oracle/_ref only here)
 # --------------------------------------------------------------------------
 def oracle_sampler(w, seed):
     from oracle import redblue as rb
@@ -231,7 +251,7 @@ def _ref_logp_row(x):
 
 
 def import_reference():
-    """The unmodified reference package from baseline/_ref (see baseline/make_ref.py), or None."""
+    """The unmodified reference package from oracle/_ref (see oracle/make_ref.py), or None."""
     if not os.path.exists(REF_ZIP):
         return None
     if REF_ZIP not in sys.path:
@@ -279,7 +299,7 @@ def time_reference(w, steps, warmup, pool_steps, repeats=3):
         ncores = host_cores()
         with one_blas_thread, mp.get_context("fork").Pool(ncores) as pool:
             s = emcee.EnsembleSampler(N, D, _ref_logp_row, moves=mv, pool=pool)
-            s.run_mcmc(w["p0"], 1, **kw)
+            s.run_mcmc(w["p0"], max(1, warmup), **kw)
             ts = []
             for _ in range(repeats):
                 t0 = time.perf_counter()
@@ -290,21 +310,24 @@ def time_reference(w, steps, warmup, pool_steps, repeats=3):
     return out
 
 
-def cpu_arms(w, steps, warmup, pool_steps):
+def cpu_arms(w, steps, warmup, pool_steps, keep_going=True):
     """The CPU baseline object: the unmodified reference (best of its two own execution modes) when
-    baseline/_ref travelled with the snapshot, with the oracle port beside it; else the port alone."""
-    port_v, port_dt = time_oracle(w, steps, max(1, min(warmup, 2)))
+    oracle/_ref holds it, with the oracle port beside it; else the port alone, named as such.  A failing
+    reference is reported in the object when `keep_going` (the GPU arm's line), else raised."""
+    port_v, port_dt = time_oracle(w, steps, warmup)
     ref = None
     try:
-        ref = time_reference(w, steps, max(1, min(warmup, 2)), pool_steps)
-    except Exception as e:  # never lose the headline over the baseline
-        ref = {"error": repr(e)}
+        ref = time_reference(w, steps, warmup, pool_steps)
+    except Exception as e:
+        if not keep_going:
+            raise
+        ref = {"error": repr(e)}  # never lose the GPU headline over the baseline beside it
     what = "%dx%d %s" % (w["nwalkers"], w["ndim"], w["name"])
     if ref and "vectorize" in ref:
         best_mode = max((k for k in ("vectorize", "pool") if k in ref), key=lambda k: ref[k]["value"])
         return {
             "value": ref[best_mode]["value"], "unit": "walker-steps/s", "cores": host_cores(), "kind": "reference",
-            "sample": "unmodified dfm/emcee@8ab6c0f (baseline/_ref), %s: vectorize=True %d steps x3 (median %.2f s, BLAS threads=%d)%s; "
+            "sample": "unmodified dfm/emcee@8ab6c0f (oracle/_ref), %s: vectorize=True %d steps x3 (median %.2f s, BLAS threads=%d)%s; "
                       "best mode = %s; numpy oracle port beside it" % (
                           what, ref["vectorize"]["steps"], ref["vectorize"]["seconds"], blas_threads(),
                           "; Pool(%d) per-walker log-prob, BLAS threads=1, %d steps x3 (median %.2f s)" % (
@@ -316,24 +339,28 @@ def cpu_arms(w, steps, warmup, pool_steps):
         }
     return {"value": port_v, "unit": "walker-steps/s", "cores": blas_threads(), "kind": "port",
             "sample": "%d steps of %s on the numpy oracle port (%.1f s; BLAS threads=%d, rest single-threaded); "
-                      "baseline/_ref absent: %s" % (steps, what, port_dt, blas_threads(), (ref or {}).get("error", "not packaged")),
+                      "unmodified reference not timed: %s" % (
+                          steps, what, port_dt, blas_threads(),
+                          (ref or {}).get("error", "oracle/_ref/emcee_reference.zip absent (oracle/make_ref.py found no "
+                                                   "readable reference checkout)")),
             "port": port_v}
 
 
 def run_reference(args, dist):
     """``--impl reference``: the reference's own CPU implementation of the path on this box's host
-    cores.  Rank 0 only."""
+    cores, every arm timed over exactly ``--steps`` steps after ``--warmup`` (the Pool arm too, unless
+    ``--cpu-pool-steps 0`` skips it).  Rank 0 only."""
     if dist.rank != 0:
         return
     w = make_workload(args.workload, args.nwalkers, args.ndim)
-    steps = max(1, min(args.steps, args.cpu_steps))
+    steps = args.steps
     t0 = time.perf_counter()
-    cpu = cpu_arms(w, steps, args.warmup, args.cpu_pool_steps)
+    cpu = cpu_arms(w, steps, args.warmup, steps if args.cpu_pool_steps > 0 else 0, keep_going=False)
     value = cpu["value"]
     line = {
         "impl": "reference",
         "metric": METRIC, "value": value, "unit": "walker-steps/s", "n_gpus": args.gpus,
-        "steps": steps, "warmup": max(1, min(args.warmup, 2)), "ms_per_step": 1e3 * w["nwalkers"] / value,
+        "steps": steps, "warmup": args.warmup, "ms_per_step": 1e3 * w["nwalkers"] / value,
         "higher_is_better": True, "scaling": "strong", "vs_baseline": None, "dtype": "f64",
         "data": "synthetic", "config": workload_config(args, w, 1, w["nwalkers"], "strong"),
         "cpu_baseline": cpu,
@@ -403,9 +430,10 @@ def build_sampler(args, w, dist, gather_results=True, pinned=False):
     return s
 
 
-def measure_device(args, w, dist, steps, warmup, flush, clocks=None):
+def measure_device(args, w, dist, steps, warmup, flush, clocks=None, dump_dir=None):
     """Device-resident throughput: CUDA events on the engine's stream around exactly `steps` steps
-    (per-step brackets with an L2 flush before each when `flush`), max over ranks."""
+    (per-step brackets with an L2 flush before each when `flush`), max over ranks.  With `dump_dir`, the
+    state after those steps is written there (rank 0)."""
     s = build_sampler(args, w, dist)
     eng = s._engine
     eng.set_option("l2_flush", 1 if flush else 0)
@@ -422,6 +450,12 @@ def measure_device(args, w, dist, steps, warmup, flush, clocks=None):
     ck = clocks.stop() if clocks is not None else None
     ms, launches = eng.last_step_timing()
     ms, wall = dist.max(ms), dist.max(wall)
+    if dump_dir is not None:
+        # read before the clock probe below steps the ensemble further; collective on a sharded engine
+        coords, log_prob = eng.get_state()
+        naccepted = eng.naccepted()
+        if dist.rank == 0:
+            dump_outputs(dump_dir, coords, log_prob, naccepted)
     out = {"ms": ms, "wall": wall, "launches": launches, "kernel": eng.last_kernel_name(),
            "value": w["nwalkers"] * steps / (ms * 1e-3)}
     if ck is not None:
@@ -561,7 +595,8 @@ def run_b200(args, dist):
 
     # ---- headline: the metric configuration, sharded over the ranks (strong scaling) -------------
     parity = parity_check(args, w, dist) if world > 1 else None
-    head = measure_device(args, w, dist, args.steps, args.warmup, args.l2_flush, ClockSampler(dist.local_rank))
+    head = measure_device(args, w, dist, args.steps, args.warmup, args.l2_flush, ClockSampler(dist.local_rank),
+                          dump_dir=args.dump_outputs)
     e2e = measure_e2e(args, w, dist, args.steps, args.warmup)
 
     # ---- weak scaling beside it: the same walkers PER GPU ----------------------------------------
@@ -645,9 +680,18 @@ def main():
     ap.add_argument("--no-stagger", action="store_true", help="dense_dmma: all pairs request their first tile at once")
     ap.add_argument("--no-pdl", action="store_true", help="dense_dmma: plain stream-ordered launches instead of programmatic dependent launches")
     ap.add_argument("--dmma-group", type=int, default=0, help="half-steps per persistent dense_dmma launch (0: library default)")
-    ap.add_argument("--cpu-steps", type=int, default=20)
-    ap.add_argument("--cpu-pool-steps", type=int, default=2, help="steps of the reference's Pool arm (0: skip it)")
+    ap.add_argument("--cpu-steps", type=int, default=20, help="steps of the cpu_baseline object beside the GPU arm")
+    ap.add_argument("--cpu-pool-steps", type=int, default=2,
+                    help="steps of the reference's Pool arm in that object (0: skip it; with --impl reference the "
+                         "Pool arm times --steps steps, and 0 skips it)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the state the timed steps of the headline run left as DIR/<name>.npy, so that two "
+                         "builds can be compared output for output (the inputs are seeded)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "b200":
+        ap.error("--dump-outputs writes what the timed GPU path computed; it needs --impl b200")
     args.warmup = max(3, args.warmup)
     args.l2_note = (
         "L2 flushed between timed steps (256 MiB device memset, outside the per-step CUDA-event brackets)"

@@ -4,7 +4,8 @@
 Run in the authoring container only (``/root/reference`` does not exist on the
 GPU box):
 
-    python -m oracle.gen_golden
+    python -m oracle.gen_golden                  # every case
+    python -m oracle.gen_golden integration      # one case (or several, by name)
 
 What it does: imports dfm/emcee from ``/root/reference/src`` (stubbing the
 setuptools_scm-generated ``emcee.emcee_version`` module that
@@ -182,6 +183,40 @@ def run_case(emcee, name, nwalkers, ndim, target, moves, p0, nsteps, seed):
     )
 
 
+INTEGRATION = os.path.join(OUT, "integration", "stretch_dense_512x16.npz")
+
+
+def integration_case(emcee):
+    """What ``tests/test_gpu_integration.py`` checks the engine against: the reference's own
+    ``EnsembleSampler.run_mcmc`` loop and ``Backend`` with its own ``StretchMove`` (``vectorize=True``),
+    512 walkers of the 16-D dense Gaussian, 25 steps, Philox key 0x1B200.  The full chain (1.6 MB) is
+    not stored: per step the SHA-256 of the chain's bytes, plus the chain of a fixed sample of 32
+    walkers, every log-probability and the per-walker acceptance counts."""
+    import hashlib
+
+    from . import targets as T
+    from .philox import PhiloxRandom
+
+    N, D, steps, seed = 512, 16, 25, 0x1B200
+    target, p0 = T.make_config("gauss_dense", N, D)
+    sampler = emcee.EnsembleSampler(N, D, target, moves=emcee.moves.StretchMove(), vectorize=True)
+    sampler._random = PhiloxRandom(seed)  # ensemble.py:166
+    sampler.run_mcmc(p0, steps, skip_initial_state_check=True)
+    chain = sampler.get_chain()
+    walkers = np.sort(np.random.default_rng(0x1B200).choice(N, 32, replace=False))
+    os.makedirs(os.path.dirname(INTEGRATION), exist_ok=True)
+    np.savez_compressed(
+        INTEGRATION,
+        seed=np.array(seed, dtype=np.uint64), icov=target.icov, p0=p0, lp0=np.asarray(target(p0)),
+        chain_sha256=np.array([hashlib.sha256(np.ascontiguousarray(c).tobytes()).hexdigest() for c in chain]),
+        walkers=walkers, chain_walkers=chain[:, walkers], log_prob=sampler.get_log_prob(),
+        accepted=sampler.backend.accepted, acceptance_fraction=sampler.acceptance_fraction,
+    )
+    print("%-32s steps=%3d  acc=%.3f  bytes=%d" % (
+        "integration/" + os.path.basename(INTEGRATION), steps, sampler.acceptance_fraction.mean(),
+        os.path.getsize(INTEGRATION)))
+
+
 def philox_kat():
     """Known answers for Philox4x32-10 itself.  The three Random123 vectors
     (kat_vectors, philox4x32-10 rows) are typed in here, not computed."""
@@ -207,6 +242,8 @@ def main():
         if only and case[0] not in only:
             continue
         run_case(emcee, *case, seed=0x656D636565B200 + idx)
+    if not only or "integration" in only:
+        integration_case(emcee)
 
 
 if __name__ == "__main__":

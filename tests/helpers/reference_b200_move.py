@@ -1,13 +1,18 @@
 """The reference-side binding of INTEGRATION.md section 4, as a maintainer of dfm/emcee would add it
 (``src/emcee/moves/b200.py``): a ``RedBlueMove`` whose ``propose`` forwards to the C ABI, and a device
-log-probability usable as ``log_prob_fn``.  Imports the REFERENCE package (``emcee``) -- it must be importable
-(``baseline/_ref/emcee_reference.zip`` on ``sys.path``) -- and nothing of ``emcee_b200``'s Python layer: the
-shared library is bound with ctypes only.  Executed by ``tests/test_gpu_integration.py``."""
+log-probability usable as ``log_prob_fn``.  The shared library is bound with ctypes only -- nothing of
+``emcee_b200``'s Python layer.  ``B200StretchMove`` subclasses the REFERENCE package's ``RedBlueMove`` and
+exists only where ``emcee`` is importable; ``DeviceGaussian`` and ``propose_stretch`` need nothing but numpy.
+Executed by ``tests/test_gpu_integration.py``."""
 import ctypes as C
 import os
 
 import numpy as np
-from emcee.moves.red_blue import RedBlueMove  # the reference's own base class (moves/red_blue.py:11)
+
+try:
+    from emcee.moves.red_blue import RedBlueMove  # the reference's own base class (moves/red_blue.py:11)
+except ImportError:
+    RedBlueMove = None
 
 _LIB = os.environ.get("EMCEE_B200_LIB") or os.path.join(
     os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__)))), "emcee_b200", "libemcee_b200.so")
@@ -52,20 +57,29 @@ class DeviceGaussian(object):
             self.ctx = C.c_void_p()
 
 
-class B200StretchMove(RedBlueMove):
-    def __init__(self, a=2.0, **kwargs):
-        self.a = a
-        super(B200StretchMove, self).__init__(**kwargs)
+def propose_stretch(ctx, coords, log_prob, a=2.0, nsplits=2, randomize_split=True, live_dangerously=False):
+    """One stretch-move step of every walker on the engine ``ctx``.  ``coords`` [N, D] and ``log_prob`` [N]
+    (C-contiguous float64) are updated in place; returns the accept mask.  The defaults are RedBlueMove's."""
+    n = coords.shape[0]
+    c = np.ascontiguousarray(coords)
+    lp = np.ascontiguousarray(log_prob)
+    _check(ctx, _lib.eb_set_state(ctx, c.ctypes.data_as(_dp), lp.ctypes.data_as(_dp)))
+    mv = _EbMove(0, nsplits, int(randomize_split), int(live_dangerously), 1.0, a, np.nan, 0, 0, 0, None, 0)
+    acc = np.zeros(n, dtype=np.uint8)
+    _check(ctx, _lib.eb_step(ctx, C.byref(mv), C.c_size_t(1), C.c_uint64(1), acc.ctypes.data_as(C.POINTER(C.c_uint8))))
+    _check(ctx, _lib.eb_get_state(ctx, coords.ctypes.data_as(_dp), log_prob.ctypes.data_as(_dp)))
+    return acc.astype(bool)
 
-    def propose(self, model, state):  # moves/red_blue.py:52
-        ctx = model.log_prob_fn.f.ctx  # _FunctionWrapper.f, ensemble.py:633
-        n, d = state.coords.shape
-        c = np.ascontiguousarray(state.coords)
-        lp = np.ascontiguousarray(state.log_prob)
-        _check(ctx, _lib.eb_set_state(ctx, c.ctypes.data_as(_dp), lp.ctypes.data_as(_dp)))
-        mv = _EbMove(0, self.nsplits, int(self.randomize_split), int(self.live_dangerously), 1.0, self.a, np.nan,
-                     0, 0, 0, None, 0)
-        acc = np.zeros(n, dtype=np.uint8)
-        _check(ctx, _lib.eb_step(ctx, C.byref(mv), C.c_size_t(1), C.c_uint64(1), acc.ctypes.data_as(C.POINTER(C.c_uint8))))
-        _check(ctx, _lib.eb_get_state(ctx, state.coords.ctypes.data_as(_dp), state.log_prob.ctypes.data_as(_dp)))
-        return state, acc.astype(bool)
+
+if RedBlueMove is not None:
+
+    class B200StretchMove(RedBlueMove):
+        def __init__(self, a=2.0, **kwargs):
+            self.a = a
+            super(B200StretchMove, self).__init__(**kwargs)
+
+        def propose(self, model, state):  # moves/red_blue.py:52
+            ctx = model.log_prob_fn.f.ctx  # _FunctionWrapper.f, ensemble.py:633
+            acc = propose_stretch(ctx, state.coords, state.log_prob, self.a, self.nsplits, self.randomize_split,
+                                  self.live_dangerously)
+            return state, acc
