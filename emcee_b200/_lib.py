@@ -29,6 +29,9 @@ EB_ERR_NAN_PARAM = -12
 EB_ERR_FEW_WALKERS = -13
 EB_ERR_NAN_INITIAL = -14
 
+EB_LAUNCH_CONFIG_FIELDS = 8
+LAUNCH_KERNELS = ("none", "generic", "tma_rows", "dense_dmma")
+
 EB_COMM_ID_BYTES = 128
 EB_IPC_BLOB_BYTES = 256
 EB_COMM_ALLGATHER = 0
@@ -94,6 +97,7 @@ _SIGNATURES = {
     ),
     "eb_set_option": (C.c_int, [C.c_void_p, C.c_char_p, C.c_int64]),
     "eb_debug_timeline": (C.c_int, [C.c_void_p, C.POINTER(C.c_int64), C.c_size_t, C.POINTER(C.c_size_t)]),
+    "eb_debug_launch_config": (C.c_int, [C.c_void_p, C.POINTER(C.c_int64), C.c_size_t]),
     "eb_last_kernel_name": (C.c_char_p, [C.c_void_p]),
     "eb_microbench": (C.c_int, [C.c_int, C.c_int, _dp]),
     "eb_host_alloc": (C.c_int, [C.c_size_t, C.POINTER(C.c_void_p)]),
@@ -389,6 +393,17 @@ class Engine(object):
         )
         k = int(cnt.value)
         return dict(partners=partners[:, :k], scalar=scalar[:k], u_accept=u[:k], active=active[:k])
+
+    def launch_config(self):
+        """Launch shape of the last fused red-blue half-step (``eb_debug_launch_config``): kernel name,
+        ``width`` (walkers per tile; lanes per walker for ``generic``), ``epl``, ``own_reg``, ``warps`` and
+        ``threads`` per CTA, ``grid`` (CTAs) and ``tiles`` (active walkers for ``generic``)."""
+        out = np.zeros(EB_LAUNCH_CONFIG_FIELDS, dtype=np.int64)
+        self._check(lib().eb_debug_launch_config(self._h, out.ctypes.data_as(C.POINTER(C.c_int64)), out.size))
+        keys = ("kernel", "width", "epl", "own_reg", "warps", "threads", "grid", "tiles")
+        cfg = dict(zip(keys, (int(v) for v in out)))
+        cfg["kernel"] = LAUNCH_KERNELS[cfg["kernel"]]
+        return cfg
 
     def debug_timeline(self):
         """[SM, consumer, tile, event] cycle stamps of the last dense_dmma half-step."""

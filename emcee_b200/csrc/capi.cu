@@ -81,6 +81,8 @@ struct eb_ctx {
   int dmma_stagger = 1;
   int dmma_group = 1;  // half-steps per persistent dense_dmma launch (1: a launch per half-step)
   int pdl = 1;           // dense_dmma launches chain as programmatic dependents (1: one GPU only, 2: sharded too)
+  int grid_cap = 0;      // most CTAs of the grid-strided half-step / dense log-prob launches (0: no cap)
+  LaunchShape last_shape{};  // launch shape of the last fused half-step (eb_debug_launch_config)
   int local_first = 0;  // sharded dense_dmma: local-partner tiles first, peer barrier behind them (0 never, 1 auto, 2 always)
   bool chain_ok = false; // the last operation enqueued on the stream is a dense_dmma kernel of this run
   // multi-GPU: log_prob / accept mask / counters (and, P2P, coords) of rows owned by OTHER ranks are stale
@@ -358,11 +360,15 @@ int eb_model_set(eb_ctx* c, int kind, const double* params, size_t nparams) {
   return EB_OK;
 }
 
+// CTA count of a grid-strided launch sized `full` (a multiple of the SM count), under option "grid_cap"
+static int capped_grid(const eb_ctx* c, int full) { return c->grid_cap > 0 && c->grid_cap < full ? c->grid_cap : full; }
+
 // ---- log-prob ----------------------------------------------------------------
 // rows of x -> out with the kernel that matches the stepping path of the model
 static cudaError_t launch_logprob(eb_ctx* c, const double* x, int64_t rows, double* out) {
   if (c->allow_dmma && c->model.kind == EB_MODEL_GAUSS_DENSE && c->model.chol != nullptr)
-    return launch_logprob_dense_dmma(c->model, c->D, x, rows, out, c->status_dev, c->sm_count, c->st);
+    return launch_logprob_dense_dmma(c->model, c->D, x, rows, out, c->status_dev, capped_grid(c, 2 * c->sm_count),
+                                     c->st);
   return launch_logprob_generic(c->model, x, rows, c->D, out, c->status_dev, c->st);
 }
 
@@ -739,11 +745,12 @@ int launch_step_generic(eb_ctx* c, const eb_move& mv, uint64_t step, const int32
     c->chain_ok = false;
     bool used_tma = false;
     if (c->allow_tma && !c->debug)
-      CK(c, launch_half_step_tma(mv.kind, a, c->sm_count, c->allow_tma >= 2, c->tma_own_reg, c->st, &used_tma));
+      CK(c, launch_half_step_tma(mv.kind, a, capped_grid(c, c->sm_count), c->allow_tma >= 2, c->tma_own_reg, c->st,
+                                 &used_tma, &c->last_shape));
     if (used_tma) {
       c->last_kernel = "tma_rows";
     } else {
-      CK(c, launch_half_step_generic(mv.kind, a, c->st));
+      CK(c, launch_half_step_generic(mv.kind, a, c->st, &c->last_shape));
       c->last_kernel = "generic";
     }
     ++launches;
@@ -882,9 +889,9 @@ int flush_dmma(eb_ctx* c, const eb_move& mv, DmmaGroup& grp, uint64_t& launches)
   // (sharded ensembles: measured slower with the dependent launch -- the early CTAs only add pollers on the
   // peer flags -- so it is opt-in there: option "pdl" = 2)
   const bool pdl = c->chain_ok && grp.nhalf == 1 && (c->comm.nranks > 1 ? c->pdl >= 2 : c->pdl >= 1);
-  int grid = 0;
-  CK(c, launch_dense_dmma(a, c->descs_host[grp.first], c->descs_dev + grp.first, grp.nhalf, bound, c->gbar, c->gbar_count, c->sm_count, pdl,
-                          &grid, c->st));
+  CK(c, launch_dense_dmma(a, c->descs_host[grp.first], c->descs_dev + grp.first, grp.nhalf, bound, c->gbar, c->gbar_count,
+                          capped_grid(c, c->sm_count), pdl, &c->last_shape, c->st));
+  const int grid = (int)c->last_shape.grid;
   c->gbar_count += (unsigned long long)(grp.nhalf - 1) * (unsigned long long)grid;
   c->last_kernel = "dense_dmma";
   c->chain_ok = grid > 0;
@@ -1456,6 +1463,11 @@ int eb_set_option(eb_ctx* c, const char* name, int64_t value) {
     c->allow_dmma = value != 0;
     return EB_OK;
   }
+  if (!strcmp(name, "grid_cap")) {
+    if (value < 0) FAIL(c, EB_ERR_INVALID, "grid_cap must be >= 0");
+    c->grid_cap = (int)std::min<int64_t>(value, 1 << 30);
+    return EB_OK;
+  }
   FAIL(c, EB_ERR_INVALID, "eb_set_option: unknown option '%s'", name);
 }
 
@@ -1481,6 +1493,13 @@ int eb_debug_taps(eb_ctx* c, int64_t* partners, double* scalar, double* u_accept
   if (u_accept) CK(c, cudaMemcpy(u_accept, c->tap_u, N * sizeof(double), cudaMemcpyDeviceToHost));
   if (active) CK(c, cudaMemcpy(active, c->tap_active, N * sizeof(int64_t), cudaMemcpyDeviceToHost));
   if (nactive) *nactive = c->tap_count;
+  return EB_OK;
+}
+
+int eb_debug_launch_config(const eb_ctx* c, int64_t* out, size_t n) {
+  if (!c || !out || n < EB_LAUNCH_CONFIG_FIELDS) return EB_ERR_INVALID;
+  static_assert(sizeof(LaunchShape) == EB_LAUNCH_CONFIG_FIELDS * sizeof(int64_t), "one int64 per field");
+  memcpy(out, &c->last_shape, sizeof(LaunchShape));
   return EB_OK;
 }
 

@@ -594,7 +594,7 @@ __global__ void __launch_bounds__(256) logprob_dense_dmma_kernel(const ModelDev 
 }
 
 template <int KB>
-cudaError_t launch_lp_t(const ModelDev& m, const double* x, int64_t rows, double* out, int* status, int sm_count,
+cudaError_t launch_lp_t(const ModelDev& m, const double* x, int64_t rows, double* out, int* status, int max_grid,
                         cudaStream_t st) {
   const size_t smem = ((size_t)packed_blocks(KB) * 32 + 8 * KB) * sizeof(double) + sizeof(uint64_t);
   const bool has_mean = m.s0 != 0.0;
@@ -605,15 +605,15 @@ cudaError_t launch_lp_t(const ModelDev& m, const double* x, int64_t rows, double
   }
   if (rows <= 0) return cudaSuccess;
   const int64_t want = (((rows + 7) >> 3) + 7) / 8;
-  const int grid = (int)(want < 2 * sm_count ? want : 2 * sm_count);
+  const int grid = (int)(want < max_grid ? want : max_grid);
   kern<<<grid, 256, smem, st>>>(m, x, rows, out, status);
   return cudaGetLastError();
 }
 
 template <int KB>
 cudaError_t launch_t(const HalfStepArgs& a, const HalfDesc& d0, const HalfDesc* descs_dev, int nhalf, int max_count,
-                     unsigned long long* gbar, unsigned long long gbar_base, int sm_count, bool pdl, int* grid_out,
-                     cudaStream_t st) {
+                     unsigned long long* gbar, unsigned long long gbar_base, int max_grid, bool pdl,
+                     LaunchShape* shape, cudaStream_t st) {
   const size_t smem = SmemLayout<KB>::total_bytes;
   const bool has_mean = a.model.s0 != 0.0;  // set by eb_model_set when mu != 0
   auto kern = has_mean ? half_step_dense_dmma_kernel<KB, true> : half_step_dense_dmma_kernel<KB, false>;
@@ -626,11 +626,10 @@ cudaError_t launch_t(const HalfStepArgs& a, const HalfDesc& d0, const HalfDesc* 
     if (e != cudaSuccess) return e;
     if (dev >= 0 && dev < 64) configured[has_mean][dev] = true;
   }
-  *grid_out = 0;
+  const int64_t ntiles = max_count > 0 ? ((int64_t)max_count + 7) / 8 : 0;
+  const int grid = (int)(ntiles < max_grid ? ntiles : max_grid);
+  *shape = LaunchShape{SHAPE_DENSE_DMMA, 8, 0, 0, DMMA_CONSUMERS, DMMA_THREADS, nhalf > 0 ? grid : 0, ntiles};
   if (max_count <= 0 || nhalf <= 0) return cudaSuccess;
-  const int64_t ntiles = ((int64_t)max_count + 7) / 8;
-  const int grid = (int)(ntiles < sm_count ? ntiles : sm_count);
-  *grid_out = grid;
   HalfStepArgs args = a;
   HalfDesc first = d0;
   if (nhalf == 1) {
@@ -682,10 +681,10 @@ void dense_dmma_pack_factor(const double* L, int D, double* packed) {
 }
 
 cudaError_t launch_logprob_dense_dmma(const ModelDev& m, int D, const double* x, int64_t rows, double* out,
-                                      int* status, int sm_count, cudaStream_t st) {
+                                      int* status, int max_grid, cudaStream_t st) {
 #define EB_LP_CASE(KB) \
   case 8 * KB:         \
-    return launch_lp_t<KB>(m, x, rows, out, status, sm_count, st);
+    return launch_lp_t<KB>(m, x, rows, out, status, max_grid, st);
   switch (D) {
     EB_LP_CASE(1)
     EB_LP_CASE(2)
@@ -709,11 +708,11 @@ cudaError_t launch_logprob_dense_dmma(const ModelDev& m, int D, const double* x,
 }
 
 cudaError_t launch_dense_dmma(const HalfStepArgs& a, const HalfDesc& d0, const HalfDesc* descs_dev, int nhalf,
-                              int max_count, unsigned long long* gbar, unsigned long long gbar_base, int sm_count,
-                              bool pdl, int* grid_out, cudaStream_t st) {
+                              int max_count, unsigned long long* gbar, unsigned long long gbar_base, int max_grid,
+                              bool pdl, LaunchShape* shape, cudaStream_t st) {
 #define EB_DMMA_CASE(KB) \
   case 8 * KB:           \
-    return launch_t<KB>(a, d0, descs_dev, nhalf, max_count, gbar, gbar_base, sm_count, pdl, grid_out, st);
+    return launch_t<KB>(a, d0, descs_dev, nhalf, max_count, gbar, gbar_base, max_grid, pdl, shape, st);
   switch (a.D) {
     EB_DMMA_CASE(1)
     EB_DMMA_CASE(2)

@@ -82,6 +82,19 @@ constexpr int MOVE_PRECOMPUTED = 100;
 
 struct Engine;  // defined in capi.cu
 
+// launch shape of one fused half-step, as eb_debug_launch_config reports it (field order = the ABI's)
+enum : int { SHAPE_NONE = 0, SHAPE_GENERIC = 1, SHAPE_TMA_ROWS = 2, SHAPE_DENSE_DMMA = 3 };
+struct LaunchShape {
+  int64_t kernel;   // SHAPE_*
+  int64_t width;    // tma_rows / dense_dmma: walkers per tile; generic: lanes per walker
+  int64_t epl;      // tma_rows: 8 on the register path, else 0
+  int64_t own_reg;  // tma_rows: own row in registers
+  int64_t warps;    // tma_rows: warps per CTA; dense_dmma: consumer warps per CTA; generic: threads / 32
+  int64_t threads;  // threads per CTA
+  int64_t grid;     // CTAs
+  int64_t tiles;    // tiles of the half-step (generic: active walkers, one per lane group)
+};
+
 // ---- kernel launchers (implemented in the .cu files) ----------------------
 // ranges (nullable): [nsteps_chunk, MAX_SPLITS] int2 = active ranks of each set owned by walkers [w_lo, w_hi)
 cudaError_t launch_split_tables(int32_t* order, const StepInfo* info_dev, int nsteps_chunk, int64_t N,
@@ -94,12 +107,15 @@ cudaError_t launch_split_tables(int32_t* order, const StepInfo* info_dev, int ns
 cudaError_t launch_locality_tables(const int32_t* order, const StepInfo* info_dev, const int2* ranges, int nsteps_chunk,
                                    int64_t N, uint64_t seed, uint64_t step0, int64_t rows_per_rank, int rank,
                                    int front_cap, int32_t* aperm, cudaStream_t st);
-cudaError_t launch_half_step_generic(int move_kind, const HalfStepArgs& a, cudaStream_t st);
+// shape (nullable): receives the launch shape
+cudaError_t launch_half_step_generic(int move_kind, const HalfStepArgs& a, cudaStream_t st,
+                                     LaunchShape* shape = nullptr);
 // TMA row-gather variant for the HBM-bound models (tma_rows.cu); *used == false: not applicable, use the generic one
 // (long_rows: also take rows so long that only one walker per tile fits; own_reg: stretch rows of <= 512 bytes keep
-// the own row in registers -- plain loads / stores -- and stage only the partner rows)
-cudaError_t launch_half_step_tma(int move_kind, const HalfStepArgs& a, int sm_count, bool long_rows, bool own_reg,
-                                 cudaStream_t st, bool* used);
+// the own row in registers -- plain loads / stores -- and stage only the partner rows).  max_grid: most CTAs of the
+// grid-strided launch (the SM count, or less to give each warp more tiles).  *shape: the launch shape when used.
+cudaError_t launch_half_step_tma(int move_kind, const HalfStepArgs& a, int max_grid, bool long_rows, bool own_reg,
+                                 cudaStream_t st, bool* used, LaunchShape* shape);
 cudaError_t launch_logprob_generic(const ModelDev& m, const double* x, int64_t rows, int D, double* out,
                                    int* status, cudaStream_t st);
 // specialised: stretch + dense Gaussian on FP64 tensor cores (DMMA).  Returns
@@ -107,9 +123,10 @@ cudaError_t launch_logprob_generic(const ModelDev& m, const double* x, int64_t r
 bool dense_dmma_supported(int D);
 size_t dense_dmma_factor_doubles(int D);
 void dense_dmma_pack_factor(const double* L, int D, double* packed);  // host
-// log-probability of dense-Gaussian rows on the tensor pipe (same arithmetic as the half-step kernel)
+// log-probability of dense-Gaussian rows on the tensor pipe (same arithmetic as the half-step kernel);
+// max_grid: most CTAs of the grid-strided launch
 cudaError_t launch_logprob_dense_dmma(const ModelDev& m, int D, const double* x, int64_t rows, double* out,
-                                      int* status, int sm_count, cudaStream_t st);
+                                      int* status, int max_grid, cudaStream_t st);
 // one half-step of a persistent dense_dmma launch
 struct HalfDesc {
   uint64_t step;       // sampler step index (Philox counter)
@@ -121,11 +138,12 @@ struct HalfDesc {
 // a.order / a.range point at the chunk's table bases; d0 == descs[0] travels by value.  max_count bounds the active ranks per
 // half-step (grid sizing).  gbar is a monotonic global counter, gbar_base its value at launch.
 // `pdl`: launch as a programmatic dependent of the previous kernel in the stream (nhalf == 1 only; the caller
-// guarantees that kernel is a dense_dmma launch of the same run).
+// guarantees that kernel is a dense_dmma launch of the same run).  max_grid: most CTAs (at most the SM count:
+// a cooperative launch needs every CTA resident).
 cudaError_t launch_dense_dmma(const HalfStepArgs& a, const HalfDesc& d0, const HalfDesc* descs_dev, int nhalf,
                               int max_count,
-                              unsigned long long* gbar, unsigned long long gbar_base, int sm_count, bool pdl,
-                              int* grid_out, cudaStream_t st);
+                              unsigned long long* gbar, unsigned long long gbar_base, int max_grid, bool pdl,
+                              LaunchShape* shape, cudaStream_t st);
 
 // ---- proposal generators of WalkMove / GaussianMove (moves_extra.cu) ----------------------------
 // acc = [S1 | S2] moment sums about a shift over n rows -> cov (np.cov) -> thresholded lower Cholesky factor L

@@ -357,7 +357,7 @@ __global__ void __launch_bounds__(256) half_step_generic_kernel(const HalfStepAr
 }
 
 template <int MOVE, int MODEL>
-static cudaError_t launch_generic_t(const HalfStepArgs& a, cudaStream_t st) {
+static cudaError_t launch_generic_t(const HalfStepArgs& a, cudaStream_t st, LaunchShape* shape) {
   const int G = lanes_per_walker(a.D);
   constexpr int NROWS = (MOVE == EB_MOVE_SNOOKER ? 4 : 1) + (MODEL == EB_MODEL_GAUSS_DENSE ? 1 : 0);
   int threads = 256;
@@ -369,8 +369,9 @@ static cudaError_t launch_generic_t(const HalfStepArgs& a, cudaStream_t st) {
   if (smem > 200 * 1024) return cudaErrorInvalidConfiguration;
   const int groups = threads / G;
   const int64_t count = (int64_t)a.i_hi - a.i_lo;
+  const unsigned grid = count > 0 ? (unsigned)((count + groups - 1) / groups) : 0u;
+  if (shape) *shape = LaunchShape{SHAPE_GENERIC, G, 0, 0, threads / 32, threads, grid, count > 0 ? count : 0};
   if (count <= 0) return cudaSuccess;
-  const unsigned grid = (unsigned)((count + groups - 1) / groups);
   auto kern = half_step_generic_kernel<MOVE, MODEL>;
   if (smem > 48 * 1024) {
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
@@ -381,30 +382,30 @@ static cudaError_t launch_generic_t(const HalfStepArgs& a, cudaStream_t st) {
 }
 
 template <int MOVE>
-static cudaError_t launch_generic_m(const HalfStepArgs& a, cudaStream_t st) {
+static cudaError_t launch_generic_m(const HalfStepArgs& a, cudaStream_t st, LaunchShape* shape) {
   switch (a.model.kind) {
     case EB_MODEL_GAUSS_ISO:
-      return launch_generic_t<MOVE, EB_MODEL_GAUSS_ISO>(a, st);
+      return launch_generic_t<MOVE, EB_MODEL_GAUSS_ISO>(a, st, shape);
     case EB_MODEL_GAUSS_DENSE:
-      return launch_generic_t<MOVE, EB_MODEL_GAUSS_DENSE>(a, st);
+      return launch_generic_t<MOVE, EB_MODEL_GAUSS_DENSE>(a, st, shape);
     case EB_MODEL_ROSENBROCK:
-      return launch_generic_t<MOVE, EB_MODEL_ROSENBROCK>(a, st);
+      return launch_generic_t<MOVE, EB_MODEL_ROSENBROCK>(a, st, shape);
     case EB_MODEL_RING:
-      return launch_generic_t<MOVE, EB_MODEL_RING>(a, st);
+      return launch_generic_t<MOVE, EB_MODEL_RING>(a, st, shape);
   }
   return cudaErrorInvalidValue;
 }
 
-cudaError_t launch_half_step_generic(int move_kind, const HalfStepArgs& a, cudaStream_t st) {
+cudaError_t launch_half_step_generic(int move_kind, const HalfStepArgs& a, cudaStream_t st, LaunchShape* shape) {
   switch (move_kind) {
     case EB_MOVE_STRETCH:
-      return launch_generic_m<EB_MOVE_STRETCH>(a, st);
+      return launch_generic_m<EB_MOVE_STRETCH>(a, st, shape);
     case EB_MOVE_DE:
-      return launch_generic_m<EB_MOVE_DE>(a, st);
+      return launch_generic_m<EB_MOVE_DE>(a, st, shape);
     case EB_MOVE_SNOOKER:
-      return launch_generic_m<EB_MOVE_SNOOKER>(a, st);
+      return launch_generic_m<EB_MOVE_SNOOKER>(a, st, shape);
     case MOVE_PRECOMPUTED:
-      return launch_generic_m<MOVE_PRECOMPUTED>(a, st);
+      return launch_generic_m<MOVE_PRECOMPUTED>(a, st, shape);
   }
   return cudaErrorInvalidValue;
 }

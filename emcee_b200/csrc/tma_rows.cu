@@ -432,8 +432,8 @@ __global__ void __launch_bounds__(TMA_MAX_THREADS, 1) half_step_tma_kernel(const
 }
 
 template <int MOVE, int MODEL>
-cudaError_t launch_tma_t(const HalfStepArgs& a, int sm_count, bool long_rows, bool own_rows_in_registers, cudaStream_t st,
-                         bool* used) {
+cudaError_t launch_tma_t(const HalfStepArgs& a, int max_grid, bool long_rows, bool own_rows_in_registers, cudaStream_t st,
+                         bool* used, LaunchShape* shape) {
   constexpr int NR = RowsPerWalker<MOVE>::value;
   *used = false;
   const int D = a.D;
@@ -468,6 +468,10 @@ cudaError_t launch_tma_t(const HalfStepArgs& a, int sm_count, bool long_rows, bo
   const int nr_smem = NR - (own_reg ? 1 : 0);
   const size_t smem = (size_t)nwarps * warp_bytes(R) / NR * nr_smem + (size_t)nwarps * 2 * sizeof(uint64_t);
   const int64_t count = (int64_t)a.i_hi - a.i_lo;
+  const int64_t ntiles = count > 0 ? (count + R - 1) / R : 0;
+  const int64_t want = (ntiles + nwarps - 1) / nwarps;
+  const int grid = (int)(want < max_grid ? want : max_grid);
+  *shape = LaunchShape{SHAPE_TMA_ROWS, R, epl8 ? 8 : 0, own_reg ? 1 : 0, nwarps, 32 * nwarps, grid, ntiles};
   if (count <= 0) {
     *used = true;
     return cudaSuccess;
@@ -479,23 +483,21 @@ cudaError_t launch_tma_t(const HalfStepArgs& a, int sm_count, bool long_rows, bo
   }
   cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return e;
-  const int64_t ntiles = (count + R - 1) / R;
-  const int64_t want = (ntiles + nwarps - 1) / nwarps;
-  const int grid = (int)(want < sm_count ? want : sm_count);
   kern<<<grid, 32 * nwarps, smem, st>>>(a, R);
   *used = true;
   return cudaGetLastError();
 }
 
 template <int MOVE>
-cudaError_t launch_tma_m(const HalfStepArgs& a, int sm_count, bool long_rows, bool own_reg, cudaStream_t st, bool* used) {
+cudaError_t launch_tma_m(const HalfStepArgs& a, int max_grid, bool long_rows, bool own_reg, cudaStream_t st, bool* used,
+                         LaunchShape* shape) {
   switch (a.model.kind) {
     case EB_MODEL_GAUSS_ISO:
-      return launch_tma_t<MOVE, EB_MODEL_GAUSS_ISO>(a, sm_count, long_rows, own_reg, st, used);
+      return launch_tma_t<MOVE, EB_MODEL_GAUSS_ISO>(a, max_grid, long_rows, own_reg, st, used, shape);
     case EB_MODEL_ROSENBROCK:
-      return launch_tma_t<MOVE, EB_MODEL_ROSENBROCK>(a, sm_count, long_rows, own_reg, st, used);
+      return launch_tma_t<MOVE, EB_MODEL_ROSENBROCK>(a, max_grid, long_rows, own_reg, st, used, shape);
     case EB_MODEL_RING:
-      return launch_tma_t<MOVE, EB_MODEL_RING>(a, sm_count, long_rows, own_reg, st, used);
+      return launch_tma_t<MOVE, EB_MODEL_RING>(a, max_grid, long_rows, own_reg, st, used, shape);
   }
   *used = false;  // dense Gaussian outside the DMMA envelope: CUDA-core generic kernel
   return cudaSuccess;
@@ -505,15 +507,15 @@ cudaError_t launch_tma_m(const HalfStepArgs& a, int sm_count, bool long_rows, bo
 
 // Tries the TMA row-gather kernel; *used tells whether it took the half-step (otherwise the
 // caller falls back to half_step_generic_kernel).
-cudaError_t launch_half_step_tma(int move_kind, const HalfStepArgs& a, int sm_count, bool long_rows, bool own_reg,
-                                 cudaStream_t st, bool* used) {
+cudaError_t launch_half_step_tma(int move_kind, const HalfStepArgs& a, int max_grid, bool long_rows, bool own_reg,
+                                 cudaStream_t st, bool* used, LaunchShape* shape) {
   switch (move_kind) {
     case EB_MOVE_STRETCH:
-      return launch_tma_m<EB_MOVE_STRETCH>(a, sm_count, long_rows, own_reg, st, used);
+      return launch_tma_m<EB_MOVE_STRETCH>(a, max_grid, long_rows, own_reg, st, used, shape);
     case EB_MOVE_DE:
-      return launch_tma_m<EB_MOVE_DE>(a, sm_count, long_rows, own_reg, st, used);
+      return launch_tma_m<EB_MOVE_DE>(a, max_grid, long_rows, own_reg, st, used, shape);
     case EB_MOVE_SNOOKER:
-      return launch_tma_m<EB_MOVE_SNOOKER>(a, sm_count, long_rows, own_reg, st, used);
+      return launch_tma_m<EB_MOVE_SNOOKER>(a, max_grid, long_rows, own_reg, st, used, shape);
   }
   *used = false;
   return cudaErrorInvalidValue;

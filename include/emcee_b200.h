@@ -205,6 +205,15 @@ int eb_last_step_timing(const eb_ctx* ctx, double* ms, uint64_t* launches);
  * (x3 for partners); *nactive returns the count. */
 int eb_debug_taps(eb_ctx* ctx, int64_t* partners, double* scalar, double* u_accept,
                   int64_t* active, int64_t* nactive);
+/* launch shape of the LAST fused red-blue half-step (test hook: which kernel
+ * variant ran), out[EB_LAUNCH_CONFIG_FIELDS] = { kernel (0 none yet, 1 generic,
+ * 2 tma_rows, 3 dense_dmma), walkers per tile (tma_rows, dense_dmma) or lanes
+ * per walker (generic), elements per lane of the tma_rows register path (8, or
+ * 0 for the run-time path), own row in registers (tma_rows, 0/1), warps per CTA
+ * (dense_dmma: consumer warps), threads per CTA, CTAs, tiles of the half-step
+ * (generic: active walkers) }.  n < EB_LAUNCH_CONFIG_FIELDS -> EB_ERR_INVALID. */
+#define EB_LAUNCH_CONFIG_FIELDS 8
+int eb_debug_launch_config(const eb_ctx* ctx, int64_t* out, size_t n);
 /* per-tile cycle stamps of the dense_dmma consumers during the LAST half-step
  * launched (option "dmma_timeline"): [SM][8 consumers][8 tiles][6 events]. */
 int eb_debug_timeline(eb_ctx* ctx, int64_t* out, size_t capacity, size_t* written);
@@ -220,7 +229,10 @@ int eb_debug_timeline(eb_ctx* ctx, int64_t* out, size_t capacity, size_t* writte
  * partner is local and take the peer barrier behind them; 0 never (default: the measured effect changes sign with the
  * number of GPUs), 1 when a consumer warp has at most two tiles per half-step, 2 always), "moments_every" (n >= 0: see
  * eb_moments; setting it resets the accumulators), "dmma_timeline" (0/1: record consumer cycle stamps
- * for eb_debug_timeline), "l2_flush"
+ * for eb_debug_timeline), "grid_cap" (n >= 0: at most n CTAs for the grid-strided launches sized by the SM count --
+ * the tma_rows and dense_dmma half-steps and the dense_dmma log-probability -- so each warp works through more
+ * tiles; results do not depend on it (draws are keyed by active rank, tiles are dealt by stride); 0 = no cap,
+ * the default), "l2_flush"
  * (0/1: benchmark hygiene -- write a 256 MiB buffer before every step and time
  * each step with its own CUDA-event pair, so eb_last_step_timing excludes the
  * flush). */

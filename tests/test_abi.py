@@ -33,6 +33,11 @@ def test_abi_version():
     assert _lib.lib().eb_abi_version() == 2
 
 
+def test_launch_config_needs_a_context_and_room_for_every_field():
+    out = (ctypes.c_int64 * _lib.EB_LAUNCH_CONFIG_FIELDS)()
+    assert _lib.lib().eb_debug_launch_config(None, out, len(out)) == _lib.EB_ERR_INVALID
+
+
 def test_eb_move_layout_matches_header():
     # ABI 2: kind, nsplits, randomize_split, live_dangerously | weight, p0, p1 | mode, reserved | seq_index | cov* | ncov
     assert ctypes.sizeof(_lib.EbMove) == 4 * 4 + 3 * 8 + 2 * 4 + 8 + 8 + 8
